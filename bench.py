@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - images/sec of the ConsistentID denoising hot path (BASELINE.json metric) on N B200s of one node.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload sd15|sdxl] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload sd15|sdxl] [--impl ours|reference] [--dump-outputs DIR]
   torchrun launches it once per GPU for N > 1 (RANK / LOCAL_RANK / WORLD_SIZE from the environment).
 
 A bench "step" = ONE pass of the hot path over one batch: the full denoising loop (UNet x 2B with the ConsistentID
@@ -252,6 +252,7 @@ def bench_workload(args, name, steps, warmup, rank, local, world):
         else:
             out = den(lat_d, pd[0], pd[1], pd[2], **kw, **ed)
         out_h.copy_(out, non_blocking=True)
+        return out_h
 
     lat_d = lat_h.to(dev); prompts_d = [p.to(dev) for p in prompts_h]; extra_d = {k: v.to(dev) for k, v in extra_h.items()}
     if use_cn:
@@ -263,23 +264,32 @@ def bench_workload(args, name, steps, warmup, rank, local, world):
     launches0 = lib.LAUNCHES
 
     def timed(fn, k):
+        """k steps of fn between CUDA events: (max over ranks of the elapsed ms, what the last step returned)."""
         cdist.barrier(); torch.cuda.synchronize()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(k):
-            fn()
+            out = fn()
         e1.record()
         torch.cuda.synchronize(); cdist.barrier()
-        return cdist.max_over_ranks(e0.elapsed_time(e1), dev)
+        return cdist.max_over_ranks(e0.elapsed_time(e1), dev), out
 
     clocks = ClockSampler(local)
     clocks.start()
-    ms_total = timed(lambda: job_resident(lat_d, prompts_d, extra_d), steps)
-    clk = clocks.stop()
+    try:
+        ms_total, out_resident = timed(lambda: job_resident(lat_d, prompts_d, extra_d), steps)
+    finally:
+        clk = clocks.stop()
     eager_calls = lib.LAUNCHES - launches0      # host-issued (non-graph) launches during the timed region
-    ms_e2e = timed(job_e2e, steps)
-    final = out_h.float()
+    ms_e2e, out_e2e = timed(job_e2e, steps)
+    final = out_e2e.float()
     finite = bool(torch.isfinite(final).all())
+    if args.dump_outputs and rank == 0:
+        # final latents of the last timed step of each path, as its caller receives them (the e2e path's land in pinned host memory)
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, f"{name}_latents.npy"), out_resident.float().cpu().numpy())
+        np.save(os.path.join(args.dump_outputs, f"{name}_e2e_latents.npy"), final.numpy())
 
     # ---- launches: kernels inside the captured per-step graphs x replays + eager launches
     per_step = None
@@ -401,8 +411,9 @@ def run_ours(args):
     names = ["sd15", "sdxl", "sdxl_b8"] if args.workload == "all" else [args.workload]
     res = None
     for i, name in enumerate(names):
-        # the headline workload runs the requested K / W; the riders a bounded K / W so that the default run stays within minutes
-        k = args.steps if i == 0 else max(1, min(args.steps, args.rider_steps))
+        # every workload times the requested K steps (the riders --rider-steps if given); the riders' warm-up is bounded so that the default run
+        # stays within minutes
+        k = args.steps if i == 0 or args.rider_steps is None else max(1, args.rider_steps)
         w = args.warmup if i == 0 else max(1, min(args.warmup, 3))
         blk = bench_workload(args, name, k, w, rank, local, world)
         if i == 0:
@@ -534,11 +545,14 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="all", choices=["all"] + list(WORKLOADS),
                     help="all = SD1.5 configs[1] headline + SDXL configs[2] + SDXL batch 8 riders in one line")
-    ap.add_argument("--rider-steps", type=int, default=4, help="timed jobs of the non-headline workloads (bounded so the default run stays within minutes)")
+    ap.add_argument("--rider-steps", type=int, default=None, help="timed jobs of the non-headline workloads (default: --steps)")
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--no-profile", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-eager", action="store_true", help="skip the eager-GPU stand-in baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps write each workload's final latents of the last timed step as DIR/<workload>_latents.npy "
+                         "(device-resident path) and DIR/<workload>_e2e_latents.npy (host-buffer path), float32; inputs and weights are seeded")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

@@ -83,8 +83,11 @@ class B200ControlNet(B200UNet):
             if li != last:
                 ops.silu_inplace(y)
             x = y
-        self._cond = (x, B, h, w)
-        return x
+        # into a persistent buffer: a captured denoising step keeps reading the address it was captured with
+        cond = self._buf("cond", tuple(x.shape))
+        cond.copy_(x)
+        self._cond = (cond, B, h, w)
+        return cond
 
     def plan(self, NB, H, W):
         if self._plan != (NB, H, W):

@@ -30,6 +30,14 @@ class B200Denoiser:
     def _dev16(self, t):
         return t.to(device=self.unet.device, dtype=self.unet.dtype, non_blocking=True)
 
+    def _persist(self, name, t, dtype=None):
+        """``t`` copied into the engine buffer ``name``.  A captured step graph reads the addresses it was captured with, so every per-call
+        tensor it reads (scheduler tables, which ``set_timesteps`` re-allocates, and caller inputs) must live at a fixed address: a fresh
+        tensor per call would leave the graph reading freed memory that the allocator hands to something else."""
+        b = self.unet._buf(name, tuple(t.shape), dtype or t.dtype)
+        b.copy_(t)
+        return b
+
     def _pair(self, neg, pos, B):
         """[2B, L, cad]: uncond rows first, then cond rows (``torch.cat([null, cond])``, :542-549)."""
         neg, pos = self._dev16(neg), self._dev16(pos)
@@ -100,7 +108,7 @@ class B200Denoiser:
             self._graphs.clear()
             self._graph_sig = sig
         sch.set_timesteps(n, device=dev)
-        coef, ts = sch.device_tables(dev)
+        coef, ts = (self._persist("sched_" + k, t) for k, t in zip(("coef", "ts"), sch.device_tables(dev)))
         if controlnet is not None:
             controlnet.set_control_image(control_image)
         phases, cn_phases = {}, {}
@@ -122,9 +130,9 @@ class B200Denoiser:
         st = {"B": B, "HW": HW, "n": n, "guidance": float(guidance_scale), "coef": coef, "ts": ts,
               "x": u._buf("lat32", (B, 4, HW), torch.float32), "x0": u._buf("lat_x0", (B, 4, HW), torch.float32),
               "x16": u._buf("lat16", (B, 4, HW)), "step": u._buf("step_dev", (1,), torch.int32),
-              "blend": torch.from_numpy(blend).to(dev), "img": image_latents.reshape(B, 4, HW).to(dev, torch.float32).contiguous(),
-              "noise": noise.reshape(B, 4, HW).to(dev, torch.float32).contiguous(),
-              "mask": mask.reshape(B, 1, HW).to(dev, torch.float32).contiguous()}
+              "blend": self._persist("blend", torch.from_numpy(blend)), "img": self._persist("img", image_latents.reshape(B, 4, HW), torch.float32),
+              "noise": self._persist("noise", noise.reshape(B, 4, HW), torch.float32),
+              "mask": self._persist("mask", mask.reshape(B, 1, HW), torch.float32)}
         st["x"].copy_(latents.reshape(B, 4, HW).to(dev, non_blocking=True))
         st["x0"].zero_(); st["step"].zero_()
         u._buf("t_dev", (1,), torch.float32).copy_(ts[:1])
@@ -213,7 +221,7 @@ class B200Denoiser:
             self._graphs.clear()
             self._graph_sig = sig
         sch.set_timesteps(n, device=dev)
-        coef, ts = sch.device_tables(dev)
+        coef, ts = (self._persist("sched_" + k, t) for k, t in zip(("coef", "ts"), sch.device_tables(dev)))
         # ---- prompt phases (K/V caches + SDXL added-cond embedding), computed once per call
         null_f = null_embeds if null_embeds_facial is None else null_embeds_facial
         phases = {}

@@ -11,10 +11,11 @@ What is restated here
 ---------------------
 * ``processors_ref``  - the reference's own code for the path:
   ``attention.py:90-174`` (Consistent_AttProcessor) and ``attention.py:177-294``
-  (Consistent_IPAttProcessor).  PINNED: ``tests/test_oracle_cpu.py``
-  imports the reference ``attention.py`` verbatim (through the 2-symbol
-  ``oracle/diffusers_shim``) and compares, and ``tests/golden/*.pt`` hold
-  outputs generated from that verbatim import (``tests/golden/make_golden.py``).
+  (Consistent_IPAttProcessor).  PINNED: ``tests/golden/*.pt`` hold outputs
+  of the reference ``attention.py`` imported verbatim (through the 2-symbol
+  ``oracle/diffusers_shim``; ``tests/golden/make_golden.py``,
+  ``tests/golden/make_pinned_golden.py``) and ``tests/test_oracle_cpu.py``
+  compares.
 * ``unet_ref`` / ``schedulers_ref`` - the third-party dependency the reference
   calls for ~99 % of the arithmetic: ``diffusers==0.23.0``
   (``requirements.txt:36``; not vendored in /root/reference, not installable

@@ -1,9 +1,9 @@
 """CPU oracle: restatement of the reference's two attention processors.
 
 TEST INFRASTRUCTURE ONLY (see oracle/__init__.py).  PINNED against the reference
-itself: tests/test_oracle_cpu.py imports /root/reference/attention.py
-verbatim (via oracle/diffusers_shim) and tests/golden/ holds outputs generated
-from it by tests/golden/make_golden.py.
+itself: tests/golden/ holds outputs of the reference attention.py imported
+verbatim (via oracle/diffusers_shim) by tests/golden/make_golden.py and
+tests/golden/make_pinned_golden.py, and tests/test_oracle_cpu.py compares.
 
 Follows:
   attention.py:90-174   Consistent_AttProcessor   (LoRA'd self-attention; without xformers

@@ -66,3 +66,19 @@ def synth_prompts(cad, seed=1, n_text=77, n_id=4, dtype=torch.float32):
 def synth_latents(b, h, w, seed=0, dtype=torch.float32, init_noise_sigma=1.0):
     g = torch.Generator().manual_seed(seed)
     return (torch.randn(b, 4, h, w, generator=g) * init_noise_sigma).to(dtype)
+
+
+def seeded_params(shapes, seed):
+    """Seeded fp32 weights for a ``[(name, shape), ...]`` state-dict layout: matrices N(0, 1/fan_in), 1-D ``*weight`` entries (LayerNorm
+    gains) 1 + 0.1 N(0, 1), other 1-D entries (biases) 0.1 N(0, 1).  Lets a golden fixture pin a module whose weights are too large to
+    store: it keeps the layout and the seed, and the test rebuilds the same weights."""
+    g = torch.Generator().manual_seed(seed)
+    out = {}
+    for name, shape in shapes:
+        if len(shape) > 1:
+            out[name] = torch.randn(shape, generator=g) * (shape[-1] ** -0.5)
+        elif name.endswith("weight"):
+            out[name] = 1.0 + 0.1 * torch.randn(shape, generator=g)
+        else:
+            out[name] = 0.1 * torch.randn(shape, generator=g)
+    return out
