@@ -214,7 +214,7 @@ int launch_gemm2_any(const CUtensorMap& a1, const CUtensorMap& a2, const CUtenso
       if (sched.tail_tiles * sp > grid) grid = sched.tail_tiles * sp;
     }
   }
-  const int flavour = g.epi == EPI_GEGLU ? EPI_GEGLU : (g.epi == EPI_QKV ? EPI_QKV : EPI_STORE);      // EPI_GELU rides on the store flavour
+  const int flavour = g.epi == EPI_GEGLU ? EPI_GEGLU : (g.epi == EPI_QKV ? EPI_QKV : EPI_STORE);      // EPI_GELU / EPI_QUICK_GELU ride on the store flavour
 #define CID_G2(S, E) (g.is_bf16 ? launch_gemm2<BN, S, E, 1>(a1, a2, b, c_out ? *c_out : b, g, grid, sched, n_tiles, st) \
                                 : launch_gemm2<BN, S, E, 0>(a1, a2, b, c_out ? *c_out : b, g, grid, sched, n_tiles, st))
   if constexpr (BN >= 32) {
@@ -229,7 +229,7 @@ int launch_gemm2_any(const CUtensorMap& a1, const CUtensorMap& a2, const CUtenso
       // whole tile ahead) at the price of a 3-stage operand ring; longer K keeps the deeper ring and one staging tile
       // lean instances (no row bias / GroupNorm statistics / GELU compiled in) for the calls that use none of them: the transformer GEMMs
 #ifndef CID_NO_LEAN_EPILOGUE
-      const bool lean = g.rowbias == nullptr && g.chan_stats == nullptr && g.epi != EPI_GELU;
+      const bool lean = g.rowbias == nullptr && g.chan_stats == nullptr && g.epi != EPI_GELU && g.epi != EPI_QUICK_GELU;
 #else
       const bool lean = false;
 #endif
@@ -421,9 +421,9 @@ int cid_gemm(const void* A, long long lda, const void* A2, long long lda2, int K
   if ((ln_stats != nullptr) != (ln_colsum != nullptr)) return fail(CID_ERR_ARG, "cid_gemm: ln_stats and ln_colsum go together");
   if (ln_stats && (reinterpret_cast<uintptr_t>(ln_stats) & 7)) return fail(CID_ERR_ARG, "cid_gemm: ln_stats must be 8-byte aligned");
   g.row_stats = row_stats; g.ln_stats = ln_stats; g.ln_colsum = ln_colsum; g.ln_eps = ln_eps; g.ln_width = K1 + K2;
-  // TMA-store epilogue (plain / GELU store flavours): 16-byte aligned rows of C and of the residual; rowbias constant inside a 128-row tile
+  // TMA-store epilogue (plain / GELU / QuickGELU store flavours): 16-byte aligned rows of C and of the residual; rowbias constant inside a 128-row tile
   CUtensorMap tc; const CUtensorMap* pc = nullptr;
-  if ((epi == CID_EPI_STORE || epi == CID_EPI_GELU) && bn >= 64 && N % 8 == 0 && ldc % 8 == 0 && (reinterpret_cast<uintptr_t>(C) & 15) == 0 &&
+  if ((epi == CID_EPI_STORE || epi == CID_EPI_GELU || epi == CID_EPI_QUICK_GELU) && bn >= 64 && N % 8 == 0 && ldc % 8 == 0 && (reinterpret_cast<uintptr_t>(C) & 15) == 0 &&
       (!residual || (ldr % 8 == 0 && (reinterpret_cast<uintptr_t>(residual) & 15) == 0))) {
     if ((rc = map_out(&tc, C, N, M, ldc))) return rc;
     pc = &tc;
@@ -484,18 +484,22 @@ int cid_conv3x3(const void* X, const void* Wt, void* Y, long long ldy, int NB, i
 }
 
 static int attn_self_impl(const void* Q, long long q_pitch, const void* K, long long k_pitch, const void* Vt, void* O, long long ldo,
-                          int B, int H, int N, int n_valid, int d, int dtype, void* stream);
+                          int B, int H, int N, int n_valid, int d, int dtype, int causal, void* stream);
 int cid_attn_self(const void* Q, long long q_pitch, const void* K, long long k_pitch, const void* Vt, void* O, long long ldo,
                   int B, int H, int N, int d, int dtype, void* stream) {
-  return attn_self_impl(Q, q_pitch, K, k_pitch, Vt, O, ldo, B, H, N, N, d, dtype, stream);
+  return attn_self_impl(Q, q_pitch, K, k_pitch, Vt, O, ldo, B, H, N, N, d, dtype, 0, stream);
+}
+int cid_attn_self_causal(const void* Q, long long q_pitch, const void* K, long long k_pitch, const void* Vt, void* O, long long ldo,
+                         int B, int H, int N, int d, int dtype, void* stream) {
+  return attn_self_impl(Q, q_pitch, K, k_pitch, Vt, O, ldo, B, H, N, N, d, dtype, 1, stream);
 }
 int cid_attn_self_ragged(const void* Q, long long q_pitch, const void* K, long long k_pitch, const void* Vt, void* O, long long ldo,
                          int B, int H, int N, int n_valid, int d, int dtype, void* stream) {
   if (n_valid <= 0 || n_valid > N) return fail(CID_ERR_ARG, "cid_attn_self_ragged: need 0 < n_valid <= N (got %d, %d)", n_valid, N);
-  return attn_self_impl(Q, q_pitch, K, k_pitch, Vt, O, ldo, B, H, N, n_valid, d, dtype, stream);
+  return attn_self_impl(Q, q_pitch, K, k_pitch, Vt, O, ldo, B, H, N, n_valid, d, dtype, 0, stream);
 }
 static int attn_self_impl(const void* Q, long long q_pitch, const void* K, long long k_pitch, const void* Vt, void* O, long long ldo,
-                          int B, int H, int N, int n_valid, int d, int dtype, void* stream) {
+                          int B, int H, int N, int n_valid, int d, int dtype, int causal, void* stream) {
   if (!Q || !K || !Vt || !O || B <= 0 || H <= 0 || N <= 0) return fail(CID_ERR_ARG, "cid_attn_self: null pointer or empty problem");
   const int dp = d_pad_for(d);
   if (dp < 0) return fail(CID_ERR_UNSUPPORTED, "cid_attn_self: head dim %d unsupported (multiple of 8, <= 160)", d);
@@ -504,12 +508,19 @@ static int attn_self_impl(const void* Q, long long q_pitch, const void* K, long 
   if ((rc = map_qk(&tq, Q, B, N, H, d, q_pitch, 128))) return rc;
   if ((rc = map_qk(&tk, K, B, N, H, d, k_pitch, 128))) return rc;
   AttnArgs a{}; a.B = B; a.H = H; a.Nq = N; a.Nkv = n_valid; a.d = d; a.scale_log2 = 1.4426950408889634f / sqrtf(float(d));
-  a.O = O; a.ldo = ldo; a.is_bf16 = dtype == CID_BF16;
+  a.O = O; a.ldo = ldo; a.is_bf16 = dtype == CID_BF16; a.causal = causal;
 #ifdef CID_ATTN_TRACE
   a.trace = g_attn_trace;
 #endif
   if ((rc = map_vt(&tv, Vt, B * H, d, N, dp))) return rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (causal) {                    // the causal mask lives in the 128-query-tile kernel only, whatever N (launch_attn_self sends N >= 256 elsewhere)
+    switch (dp) {
+#define CID_ATTN_CAUSAL(DP) case DP: return a.is_bf16 ? launch_attn_self_t<DP, 1>(tq, tk, tv, a, st) : launch_attn_self_t<DP, 0>(tq, tk, tv, a, st);
+      CID_ATTN_CAUSAL(32) CID_ATTN_CAUSAL(48) CID_ATTN_CAUSAL(64) CID_ATTN_CAUSAL(80) CID_ATTN_CAUSAL(128) CID_ATTN_CAUSAL(160)
+#undef CID_ATTN_CAUSAL
+    }
+  }
   switch (dp) {
     case 32: return launch_attn_self<32>(tq, tk, tv, a, st);
     case 48: return launch_attn_self<48>(tq, tk, tv, a, st);
@@ -697,6 +708,16 @@ int cid_silu_inplace(void* y, long long n_elems, int dtype, void* stream) {
   if (!y || n_elems % 8) return fail(CID_ERR_ARG, "cid_silu_inplace: n_elems must be a multiple of 8");
   silu_inplace_kernel<<<grid_for(n_elems / 8, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>((uint4*)y, n_elems / 8, dtype == CID_BF16);
   CID_CHECK_LAUNCH("silu_inplace_kernel");
+  return 0;
+}
+int cid_embed_tokens(const long long* ids, int B, int L, int Lp, const void* tok, long long V, const void* pos, void* out, int C, int dtype,
+                     void* stream) {
+  if (!ids || !tok || !pos || !out || B <= 0 || L <= 0 || Lp < L || V <= 0 || C <= 0 || C % 8)
+    return fail(CID_ERR_ARG, "cid_embed_tokens: need B, L, V > 0, Lp >= L and C %% 8 == 0 (B=%d L=%d Lp=%d C=%d)", B, L, Lp, C);
+  const long long total = (long long)B * Lp * (C / 8);
+  embed_tokens_kernel<<<grid_for(total, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+      ids, L, Lp, (const uint4*)tok, V, (const uint4*)pos, (uint4*)out, C / 8, total, dtype == CID_BF16);
+  CID_CHECK_LAUNCH("embed_tokens_kernel");
   return 0;
 }
 int cid_inpaint_blend(float* x, void* x16, const float* image_latents, const float* noise, const float* mask, int B, int HW,

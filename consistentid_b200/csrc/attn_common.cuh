@@ -27,6 +27,7 @@ struct AttnArgs {
   int n_text, ip_off, n_ip;   // cross: key ranges [0, n_text) and [ip_off, ip_off + n_ip)
   float ip_scale;
   int vt4d;              // V^T map is the 4-D {64 keys, d, N/64, B*H} view: both 64-key chunks of a tile in ONE TMA instruction
+  int causal;            // self (attn_self5_kernel only): query row q sees keys 0..q (CLIP text encoder); 0 for every other caller
   long long* trace;      // debug builds (-DCID_ATTN_TRACE, tools/trace_attn.py): per-tile phase timestamps of the CTAs with blockIdx.y == z == 0
 };
 

@@ -81,7 +81,8 @@ attn_self5_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
 
   const int warp = warp_id(), lane = lane_id();
   const int q0 = blockIdx.x * 128, h = blockIdx.y, b = blockIdx.z;
-  const int T = (a.Nkv + 127) / 128;
+  // causal: key tiles above the diagonal are skipped by all three roles alike (a disagreement on T would leave an mbarrier waiting forever)
+  const int T = a.causal ? min((a.Nkv + 127) / 128, int(blockIdx.x) + 1) : (a.Nkv + 127) / 128;
 
   if (warp == 0 && lane == 0) { tma_prefetch_desc(&tmQ); tma_prefetch_desc(&tmK); tma_prefetch_desc(&tmVt); }
   if (warp == 1) {
@@ -225,7 +226,10 @@ attn_self5_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant
     auto stamp = [&](int, int) {};
 #endif
     for (int j = 0; j < T; ++j) {
-      const int kvalid = a.Nkv - j * 128;
+      // keys of this tile the row may see: the ragged tail, and under the causal mask keys <= the row's own index (only the diagonal tile
+      // cuts: j < blockIdx.x gives >= 129); every row keeps key j * 128 at least, so no row sums to l = 0
+      int kvalid = a.Nkv - j * 128;
+      if (a.causal) kvalid = min(kvalid, q0 + r - j * 128 + 1);
       stamp(j, 0);
       mbar_wait(s_full, uint32_t(j & 1));
       tc_fence_after();

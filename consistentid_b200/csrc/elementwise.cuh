@@ -411,6 +411,30 @@ silu_inplace_kernel(uint4* __restrict__ y, long long total_vec, int bf) {
     y[i] = pack8(a, bf);
   }
 }
+// CLIP text embeddings: out[b*Lp + i] = tok[ids[b, i]] + pos[i] for i < L, zero rows for L <= i < Lp (fp32 sum, one rounding, as the 16-bit
+// torch add); an id outside [0, V) contributes a zero token row and is never dereferenced
+__global__ void __launch_bounds__(256)
+embed_tokens_kernel(const long long* __restrict__ ids, int L, int Lp, const uint4* __restrict__ tok, long long V, const uint4* __restrict__ pos,
+                    uint4* __restrict__ out, int CV, long long total_vec, int bf) {
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total_vec; i += (long long)gridDim.x * blockDim.x) {
+    const long long row = i / CV;
+    const int c = int(i - row * CV);
+    const int b = int(row / Lp), t = int(row - (long long)b * Lp);
+    if (t >= L) { out[i] = make_uint4(0u, 0u, 0u, 0u); continue; }
+    const long long id = ids[(long long)b * L + t];
+    float a[8], p[8];
+    unpack8(pos[(long long)t * CV + c], p, bf);
+    if (id >= 0 && id < V) {
+      unpack8(tok[id * CV + c], a, bf);
+#pragma unroll
+      for (int k = 0; k < 8; ++k) a[k] += p[k];
+      out[i] = pack8(a, bf);
+    } else {
+      out[i] = pack8(p, bf);
+    }
+  }
+}
+
 // inpaint latent blending after a scheduler step (pipelines/StableDIffusionControlNetInpaint_ConsistentID.py:437-449):
 //   x = (1 - m) * (ca * image_latents + cn * noise) + m * x,   {ca, cn} = blend_table[step] = add_noise coefficients of the
 //   NEXT timestep ((1, 0) on the last step).  x: fp32 master latents [B,4,HW]; mask [B,1,HW] (1 = repaint).

@@ -14,7 +14,7 @@
 
 namespace cid {
 
-enum EpiMode : int { EPI_STORE = 0, EPI_GEGLU = 1, EPI_QKV = 2, EPI_GELU = 3, EPI_STORE_TMA = 5, EPI_STORE_TMA2 = 6 };   // EPI_STORE_TMA2: the same with two staging tiles (residual prefetched a tile ahead)   // EPI_STORE_TMA: kernel-internal flavour (store epilogue staged through smem + TMA)   // EPI_GELU: C = gelu_erf(acc + bias) (CLIP MLP fc1)
+enum EpiMode : int { EPI_STORE = 0, EPI_GEGLU = 1, EPI_QKV = 2, EPI_GELU = 3, EPI_QUICK_GELU = 4, EPI_STORE_TMA = 5, EPI_STORE_TMA2 = 6 };   // EPI_STORE_TMA2: the same with two staging tiles (residual prefetched a tile ahead)   // EPI_STORE_TMA: kernel-internal flavour (store epilogue staged through smem + TMA)   // EPI_GELU: C = gelu_erf(acc + bias) (CLIP MLP fc1)   // EPI_QUICK_GELU: C = quick_gelu(acc + bias) (OpenAI CLIP text MLP fc1)
 enum AMode : int { A_GEMM = 0, A_CONV = 1, A_CONV_S2 = 2 };
 
 struct GemmArgs {
@@ -86,5 +86,7 @@ __device__ __forceinline__ float gelu_erf(float x) {
   const float e = 1.0f - rp;
   return 0.5f * x * (1.0f + copysignf(e, x));
 }
+// QuickGELU of the OpenAI CLIP checkpoints (hidden_act "quick_gelu"): x * sigmoid(1.702 x), fp32
+__device__ __forceinline__ float quick_gelu(float x) { return x / (1.0f + __expf(-1.702f * x)); }
 
 }  // namespace cid

@@ -594,6 +594,9 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tmA1, const __grid_constant_
                 if (!LEAN && STOREF && g.epi == EPI_GELU) {
 #pragma unroll
                   for (int j = 0; j < 16; ++j) v[j] = gelu_erf(v[j]);
+                } else if (!LEAN && STOREF && g.epi == EPI_QUICK_GELU) {
+#pragma unroll
+                  for (int j = 0; j < 16; ++j) v[j] = quick_gelu(v[j]);
                 }
                 if (STOREF && g.row_stats != nullptr) {
 #pragma unroll

@@ -12,7 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("CID_LIB_PATH") or os.path.join(_HERE, "libcidb200.so")     # CID_LIB_PATH: A/B builds of the same ABI (tools/build_variant.sh)
 
 F16, BF16 = 0, 1
-EPI_STORE, EPI_GEGLU, EPI_QKV, EPI_GELU = 0, 1, 2, 3
+EPI_STORE, EPI_GEGLU, EPI_QKV, EPI_GELU, EPI_QUICK_GELU = 0, 1, 2, 3, 4
 
 
 class CidError(RuntimeError):
@@ -61,6 +61,8 @@ _SIGS = {
     "cid_layernorm_rows": ([_vp, _ll, _ll, _ll, _vp, _vp, _vp, _ll, _ll, _ll, _ll, _ll, _i, _f, _i, _vp], _i),
     "cid_perceiver_attn": ([_vp, _ll, _vp, _ll, _vp, _ll, _i, _i, _i, _i, _i, _i, _vp], _i),
     "cid_softmax_rows": ([_vp, _ll, _ll, _i, _i, _vp], _i),
+    "cid_attn_self_causal": ([_vp, _ll, _vp, _ll, _vp, _vp, _ll, _i, _i, _i, _i, _i, _vp], _i),
+    "cid_embed_tokens": ([_vp, _i, _i, _i, _vp, _ll, _vp, _vp, _i, _i, _vp], _i),
 }
 EXPORTS = tuple(_SIGS)
 for _name, (_args, _res) in _SIGS.items():

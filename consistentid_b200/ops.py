@@ -131,6 +131,35 @@ def attn_self(q, k, vt, out, B, H, N, d, n_valid=None):
     return out
 
 
+def attn_self_causal(q, k, vt, out, B, H, N, d):
+    """attn_self under the causal mask of the CLIP text transformer: query row i attends to keys 0..i (same layouts as attn_self)."""
+    with _prof("attn_self", 2.0 * B * H * N * (N + 1) * d, 2.0 * 4 * B * N * H * d, ("B%d" % B, "H%d" % H, "N%d" % N, "d%d" % d)):
+        call("cid_attn_self_causal", _p(q), q.stride(0), _p(k), k.stride(0), _p(vt), _p(out), out.stride(0), B, H, N, d, _dt(q), _stream())
+    return out
+
+
+def embed_tokens(ids, tok, pos, out, Lp):
+    """out[b*Lp + i] = tok[ids[b, i]] + pos[i] for i < L, zero rows up to Lp.  ids: int64 [B, L]; tok [V, C], pos [>= L, C], out [B*Lp, C].
+    Host ids are range-checked (ValueError) and copied to out's device; on-device ids outside [0, V) read as zero token rows."""
+    if ids.ndim != 2 or ids.dtype != torch.int64:
+        raise TypeError(f"embed_tokens: ids must be int64 [B, L], got {ids.dtype} {tuple(ids.shape)}")
+    B, L = ids.shape
+    V, C = tok.shape
+    if L > pos.shape[0] or L > Lp:
+        raise ValueError(f"embed_tokens: {L} tokens but {pos.shape[0]} positions / {Lp} rows")
+    if ids.device.type == "cpu":
+        if ids.numel() and (int(ids.min()) < 0 or int(ids.max()) >= V):
+            raise ValueError(f"embed_tokens: token ids must lie in [0, {V}), got [{int(ids.min())}, {int(ids.max())}]")
+        ids = ids.to(out.device)
+    ids = ids.contiguous()
+    _chk(ids, "ids")
+    if tok.dtype != out.dtype or pos.dtype != out.dtype:
+        raise TypeError(f"embed_tokens: tok {tok.dtype} / pos {pos.dtype} / out {out.dtype} must match")
+    assert tok.is_contiguous() and pos.is_contiguous() and out.is_contiguous() and out.shape == (B * Lp, C)
+    call("cid_embed_tokens", _p(ids), B, L, Lp, _p(tok), V, _p(pos), _p(out), C, _dt(out), _stream())
+    return out
+
+
 def attn_cross(q, k_cat, vt_cat, out, B, H, N, d, n_text, n_ip, ip_scale):
     with _prof("attn_cross", 4.0 * B * H * N * (n_text + n_ip) * d, 2.0 * 2 * B * N * H * d, ("B%d" % B, "H%d" % H, "N%d" % N, "d%d" % d)):
         call("cid_attn_cross", _p(q), q.stride(0), _p(k_cat), _p(vt_cat), _p(out), out.stride(0), B, H, N, d, n_text, n_ip,

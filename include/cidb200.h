@@ -23,7 +23,7 @@ extern "C" {
 
 typedef enum { CID_OK = 0, CID_ERR_ARG = -1, CID_ERR_CUDA = -2, CID_ERR_UNSUPPORTED = -3, CID_ERR_DRIVER = -4 } cid_status;
 typedef enum { CID_F16 = 0, CID_BF16 = 1 } cid_dtype;
-typedef enum { CID_EPI_STORE = 0, CID_EPI_GEGLU = 1, CID_EPI_QKV = 2, CID_EPI_GELU = 3 } cid_epilogue;
+typedef enum { CID_EPI_STORE = 0, CID_EPI_GEGLU = 1, CID_EPI_QKV = 2, CID_EPI_GELU = 3, CID_EPI_QUICK_GELU = 4 } cid_epilogue;
 
 int cid_version(void);
 const char* cid_last_error(void);
@@ -45,6 +45,8 @@ int cid_gemm_tile_n(int N, int epi);
  *   epi = GEGLU : B rows interleaved per tile (value half | gate half); writes C[M, N/2] = v * gelu(g).
  *   epi = QKV   : columns >= n_split are V and are written TRANSPOSED to Vt[(row/ntok)*heads + h, dd, row%ntok].
  *   epi = GELU  : C = gelu_erf(acc + bias (+ residual)) - the fc1 + activation of the CLIP vision MLP (SURVEY 8f-4).
+ *   epi = QUICK_GELU : C = q(acc + bias (+ residual)), q(x) = x * sigmoid(1.702 x) in fp32 - the fc1 + activation of the OpenAI CLIP
+ *                 ViT-L/14 text MLP (hidden_act "quick_gelu").
  *   chan_stats  : non-NULL (plain store epilogue only) = GroupNorm statistics of the OUTPUT fused into the epilogue: per (sample, column)
  *                 sum and sum of squares are ADDED to chan_stats[(row / stats_rows) * N + col][2] (fp32, zeroed by the caller); stats_rows =
  *                 rows per sample, a multiple of 128.  Consumed by cid_gn_apply_ch: the standalone statistics pass (one re-read of the
@@ -150,6 +152,19 @@ int cid_perceiver_attn(const void* q, long long ldq, const void* kv, long long l
  * pipline_StableDiffusion_ConsistentID.py:182-183, 202-203).  Rows >= n_valid of O are computed but meaningless. */
 int cid_attn_self_ragged(const void* Q, long long q_pitch, const void* K, long long k_pitch, const void* Vt, void* O, long long ldo,
                          int B, int H, int N, int n_valid, int d, int dtype, void* stream);
+/* cid_attn_self with the causal mask of the CLIP text transformer: softmax(Q K^T / sqrt(d) + mask) V where query row q sees keys 0..q, so
+ * every row has at least one key.  Same arguments and layouts as cid_attn_self (N % 8 == 0, head dims multiple of 8 up to 160).  Runs the
+ * 128-query-tile kernel for every N; key tiles above the diagonal are never loaded.  Rows of a sequence padded from L to N tokens never read
+ * the pad keys, but pad V rows must hold finite values (masked probabilities are zeros that still multiply them). */
+int cid_attn_self_causal(const void* Q, long long q_pitch, const void* K, long long k_pitch, const void* Vt, void* O, long long ldo,
+                         int B, int H, int N, int d, int dtype, void* stream);
+
+/* ---- CLIP text encoder ---- */
+/* Token + position embedding gather: out[b*Lp + i, :] = tok[ids[b*L + i], :] + pos[i, :] for i < L, and zero rows for L <= i < Lp.
+ * ids: int64 [B, L] device array (what tokenizers return); tok: [V, C], pos: [>= L, C], out: [B*Lp, C], all 16-bit, C % 8 == 0.
+ * An id outside [0, V) is never dereferenced: it contributes a zero token row (out = pos[i]). */
+int cid_embed_tokens(const long long* ids, int B, int L, int Lp, const void* tok, long long V, const void* pos, void* out, int C, int dtype,
+                     void* stream);
 
 /* ---- VAE decode (SURVEY.md 8f-3): everything but this reuses cid_conv3x3 / cid_gemm / cid_gn_* / cid_upsample2x ---- */
 /* In-place softmax over each row of x[rows, cols] (pitch ld), fp32 math: probabilities of the single-head d=512 attention of the VAE mid
